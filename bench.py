@@ -17,6 +17,9 @@ One JSON line on stdout (rank 0).  ``value`` = whole-job heads/s with inputs res
 inside the timed region, double-buffered against the compute.  Sub-objects: ``roofline`` (dominant kernel), ``cpu_baseline``,
 ``decode_microbench`` (config 5), ``config3`` (batch 512, bf16 encoder) at N=1, ``config4`` (512 per GPU) at N>1,
 ``strict_fp32_operands``, ``parity`` (against the unmodified reference when oracle/_ref is present).
+
+``--dump-outputs DIR`` writes what the timed path returned in its last timed step as ``DIR/<name>.npy`` (float32, or float64
+for 64-bit and integer outputs), so that two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ UNIT = "heads/s"
 FLOPS_PER_IMAGE_ENCODER = 2 * 7_559_801_344        # SURVEY §8(d), analytic
 FLOPS_PER_HEAD_BLEND = 13_140_168                  # 2*15069*(400+36), as written in the reference
 BYTES_PER_HEAD_DECODE = 413 * 4 + 5023 * 3 * 4     # SURVEY §8(d): params in, vertices out
+DUMP_LIMIT_BYTES = 64 << 20
 
 # BASELINE.json `configs`, numbered 1..5 as in SURVEY §8(d)
 CONFIGS = {
@@ -147,6 +151,30 @@ class ClockSampler:
                 "samples": len(self.samples), "power_w_max": max(pw) if pw else None}
 
 
+def dump_outputs(outdir, outputs):
+    """Write each output as ``outdir/<name>.npy`` (float32, or float64 for 64-bit and integer outputs).  When they would
+    exceed DUMP_LIMIT_BYTES in all, every array keeps the same fraction of its leading-axis rows (heads), drawn with a fixed
+    seed, and the kept row indices go to ``outdir/rows_<name>.npy`` (counted in the limit)."""
+    import numpy as np
+    import torch
+    outs = {k: torch.as_tensor(t) for k, t in outputs.items()}
+    size = {k: 8 if t.element_size() > 4 or not t.is_floating_point() else 4 for k, t in outs.items()}
+    total = sum(t.numel() * size[k] for k, t in outs.items())
+    headers = 1024 * (2 * len(outs))                                 # .npy headers, generously
+    os.makedirs(outdir, exist_ok=True)
+    if total + headers > DUMP_LIMIT_BYTES:
+        cost = sum(t.numel() * size[k] + 8 * t.shape[0] for k, t in outs.items())      # data + row index, all rows
+        frac = (DUMP_LIMIT_BYTES - headers) / cost
+    for k, t in outs.items():
+        if total + headers > DUMP_LIMIT_BYTES:
+            n = t.shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * frac)), replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+            np.save(os.path.join(outdir, f"rows_{k}.npy"), rows.astype(np.float64))
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(outdir, f"{k}.npy"), a.astype(np.float64 if size[k] == 8 else np.float32))
+
+
 # ------------------------------------------------------------------------------------------------------ reference arm
 def _reference_runner(sd):
     """-> (step(x) for a [B,3,256,256] batch, description, kind).  kind "reference": the UNMODIFIED reference code
@@ -214,8 +242,10 @@ def run_reference(args):
         step(x[:8])                                       # warm-up on a slice: the timed steps below are the full batch
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step(x)
+        out = step(x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     val = B * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -231,10 +261,11 @@ def run_reference(args):
 
 # ------------------------------------------------------------------------------------------------------ our arm
 def _pipeline_timer(dist, distributed, dev):
-    """timed(stream, x, steps) -> ms for `steps` batches through a BatchStream (device events; max over ranks)."""
+    """timed(stream, x, steps) -> ms for `steps` batches through a BatchStream (device events; max over ranks).  With a
+    dict `last`, the results of the last batch are copied into it (as host tensors) after the timed region."""
     import torch
 
-    def timed(stream, x, steps):
+    def timed(stream, x, steps, last=None):
         stream.drain()
         if distributed:
             dist.barrier()
@@ -246,9 +277,13 @@ def _pipeline_timer(dist, distributed, dev):
                 stream.collect()
             stream.submit(x)
         e1.record(stream.copy_out)                      # last stage of the last batch (stages of one slot run in order)
-        stream.drain()
+        while stream._inflight:                         # drain: the final collect() returns the last batch
+            res = stream.collect()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
+        if last is not None:
+            gathered = res.pop("gathered", {})
+            last.update({k: gathered.get(k, v).cpu() for k, v in res.items()})
         if distributed:
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -312,7 +347,10 @@ def run_ours(args):
     step_eager()
     torch.cuda.synchronize()
     launches_per_step = _lib.launch_count() - launches0      # a graph replay launches the same kernels (counted at capture)
-    ms_total = timed(dev_stream, x_dev, args.steps)          # EXACTLY K steps -> `value`
+    last = {} if args.dump_outputs and rank == 0 else None
+    ms_total = timed(dev_stream, x_dev, args.steps, last)    # EXACTLY K steps -> `value`
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     # a region of >= 1.5 s of the same steps: settled clocks, enough nvidia-smi samples; reported beside the K-step number
     per_step = ms_total / args.steps
     n_long = max(args.steps, int(1500.0 / max(per_step, 1e-3)) + 1) if not args.quick else args.steps
@@ -497,9 +535,10 @@ def sub_pipeline(FaceMeshPredictor, DEFAULT_CONFIG, sd, static, local_rank, B, p
     return out
 
 
-def decode_microbench(head_mesh, dev, steps, warmup, n_total=1 << 20, fast=True, cluster=False):
+def decode_microbench(head_mesh, dev, steps, warmup, n_total=1 << 20, fast=True, cluster=False, last=None):
     """BASELINE.json configs[4]: FLAME-decode-only, `n_total` param vectors -> 5023-vertex meshes per step, streamed through a
-    fixed output ring; reports the blend-shape tensor-core roofline and the HBM-write roofline side by side."""
+    fixed output ring; reports the blend-shape tensor-core roofline and the HBM-write roofline side by side.  With a dict
+    `last`, the vertices of the last pass of the last step are copied into it after the timed region."""
     import torch
     from dad_3dheads_b200 import _lib
     from oracle.flame_oracle import sample_params                   # input generation only (outside the timed region)
@@ -511,7 +550,8 @@ def decode_microbench(head_mesh, dev, steps, warmup, n_total=1 << 20, fast=True,
 
     def step():
         for lo, hi in passes:
-            dec.decode(params[lo:hi], want_vertices=True, want_projected=False, fast=fast, cluster=cluster)
+            v3, _ = dec.decode(params[lo:hi], want_vertices=True, want_projected=False, fast=fast, cluster=cluster)
+        return v3
 
     for _ in range(max(warmup, 1)):
         step()
@@ -519,11 +559,15 @@ def decode_microbench(head_mesh, dev, steps, warmup, n_total=1 << 20, fast=True,
     l0 = _lib.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
+    for _ in range(steps - 1):
         step()
+    v3 = step()
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if last is not None:
+        last["3d_vertices"] = v3
+    del v3
     value = n_total * steps / (ms * 1e-3)
     peaks = _peaks()
     products = 1 if fast else 3
@@ -553,7 +597,11 @@ def run_decode_microbench(args):
     sampler = ClockSampler(0)
     sampler.start()
     fast = args.precision in ("fp16", "bf16")
-    d = decode_microbench(hm, dev, args.steps, max(args.warmup, 3), n_total=args.batch, fast=fast, cluster=args.decode_cluster)
+    last = {} if args.dump_outputs else None
+    d = decode_microbench(hm, dev, args.steps, max(args.warmup, 3), n_total=args.batch, fast=fast, cluster=args.decode_cluster,
+                          last=last)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     clocks = sampler.stop()
     line = {"metric": d.pop("metric"), "value": d["value"], "unit": UNIT, "n_gpus": 1, "steps": args.steps,
             "warmup": max(args.warmup, 3), "ms_per_step": d["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -615,6 +663,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="profiling aid (ncu launch lists): no >= 1.5 s region, no sub-objects, "
                     "no strict-mode run, no CPU baseline -- only warm-up + the K timed steps of both arms")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (at most 64 MB; a seeded row sample "
+                         "of larger outputs)")
     ap.add_argument("--workload", default=None, choices=["pipeline", "decode"], help="legacy alias: decode = --config 5")
     args = ap.parse_args()
     if args.workload == "decode":

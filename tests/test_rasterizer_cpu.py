@@ -1,15 +1,14 @@
 """-m "not gpu": host-side pieces of the rasteriser row (SURVEY 8f row 4) -- the CSR adjacency the GPU vertex-normal kernel walks,
-and the oracle itself: the reference's own C++ rasteriser (oracle/_ref/libsim3dr_ref.so, built from Sim3DR/lib/rasterize_kernel.cpp
-where it lies) loads, and agrees with a plain numpy restatement of its per-pixel rule on a small scene (rasterize_kernel.cpp:
-219-292: barycentric inside test, depth = weighted vertex depth, strictly-greater z test, colour = weighted vertex colours)."""
-import ctypes as C
+and the oracle itself: the output of the reference's own C++ rasteriser (Sim3DR/lib/rasterize_kernel.cpp, stored in
+tests/golden/reference_rasterizer.npz) agrees with a plain numpy restatement of its per-pixel rule on a small scene
+(rasterize_kernel.cpp:219-292: barycentric inside test, depth = weighted vertex depth, strictly-greater z test, colour = weighted
+vertex colours)."""
 import os
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SO = os.path.join(ROOT, "oracle", "_ref", "libsim3dr_ref.so")
+GOLD = os.path.join(ROOT, "tests", "golden", "reference_rasterizer.npz")
 
 
 def test_vertex_adjacency_is_the_ascending_incidence_list():
@@ -32,17 +31,19 @@ def _weights(px, py, p0, p1, p2):
     return np.array([1 - u - v, v, u], np.float32)
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_SO), reason="oracle/_ref/libsim3dr_ref.so not built (python -m oracle.build_ref)")
-def test_reference_rasteriser_matches_its_per_pixel_rule():
-    lib = C.CDLL(REF_SO)
-    lib.sim3dr_ref_rasterize.argtypes = [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_float, C.c_int]
-    h, w = 24, 28
+def small_scene():
+    """Two overlapping triangles over a 24x28 image, with per-vertex colours."""
     v = np.array([[2, 3, 1.0], [20, 4, 2.0], [6, 19, 3.0], [25, 22, 0.5], [3, 21, 5.0], [22, 2, 4.0]], np.float32)
     t = np.array([[0, 1, 2], [3, 4, 5]], np.int32)
     c = np.random.default_rng(1).random((6, 3)).astype(np.float32)
-    img = np.zeros((h, w, 3), np.uint8)
-    depth = np.zeros((h, w), np.float32) - 1e8
-    lib.sim3dr_ref_rasterize(img.ctypes.data, v.ctypes.data, t.ctypes.data, c.ctypes.data, depth.ctypes.data, 2, h, w, 3, 1.0, 0)
+    return v, t, c
+
+
+def test_reference_rasteriser_matches_its_per_pixel_rule():
+    h, w = 24, 28
+    v, t, c = small_scene()
+    z = np.load(GOLD)
+    img, depth = z["small_image"], z["small_depth"]
     want = np.zeros((h, w, 3), np.float32)
     zbuf = np.zeros((h, w), np.float32) - 1e8
     for tri in t:
